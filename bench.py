@@ -2,7 +2,7 @@
 """Benchmark of the Aurora forward hot path (BASELINE.json: forecast-steps/sec on the 0.25-degree
 721x1440x13-level configuration, B = 1, history 2; 1.3 B-parameter `Aurora`).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 * `--impl ours` (default): one "step" = one `Aurora.forward` through the sm_100a kernels.
     value : steps/s with the input Batch already resident in HBM (CUDA events, max over ranks)
@@ -131,6 +131,30 @@ def randomise_parameters_(model, seed: int = 0) -> None:
     for name, p in model.named_parameters():
         if p.dim() == 1 and ("surf_norm.weight" in name or name.endswith("norm.weight")):
             p.data.fill_(1.0)
+
+
+DUMP_MAX_BYTES = 64 * 10**6  # --dump-outputs: all .npy files together stay below this
+
+
+def dump_outputs(pred, out_dir: str) -> None:
+    """Write the prediction `pred` as float32 `out_dir/<group>_<name>.npy` (group: surf, static, atmos).  When all
+    fields together would exceed DUMP_MAX_BYTES, every field keeps the same share of its values, flattened, at sorted
+    flat indices drawn from one generator seeded with 0 in field order: two builds given the same arguments dump the
+    same points."""
+    import numpy as np
+
+    fields = {f"{grp}_{k}": v.detach() for grp, d in (("surf", pred.surf_vars), ("static", pred.static_vars),
+                                                       ("atmos", pred.atmos_vars)) for k, v in d.items()}
+    budget = DUMP_MAX_BYTES // 4 - 1024 * len(fields)  # float32 values; 4 KiB per file left for the .npy header
+    share = min(1.0, budget / sum(v.numel() for v in fields.values()))
+    g = torch.Generator().manual_seed(0)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, v in fields.items():
+        if share < 1.0:
+            idx = torch.randint(v.numel(), (int(v.numel() * share),), generator=g).unique()
+            v = v.reshape(-1)[idx.to(v.device)]
+        np.save(out / f"{name}.npy", v.float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -471,7 +495,14 @@ def main() -> None:
                     help="also time one N-step autoregressive rollout (BASELINE configs[2]: 40) and add a `rollout` object")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the prediction of the last one as DIR/<group>_<name>.npy "
+                         "(float32, a fixed sample when over 64 MB; rank 0's, i.e. its latitude band when sharded)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.warmup < 1:
         args.warmup = 1
 
@@ -540,6 +571,8 @@ def main() -> None:
     # kernels launched by this library in the timed region: eager launches + those replayed from captured graphs
     launches = (cabi.launch_count() - launches0) + (model._engine.replayed_launches - replayed0)
     ms = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(pred, args.dump_outputs)
 
     # ---- end to end through the public API from pinned host memory ----
     e2e_ms = None

@@ -22,6 +22,7 @@ from __future__ import annotations
 
 import hashlib
 import json
+import os
 import shutil
 import sys
 from pathlib import Path
@@ -36,9 +37,14 @@ def _sha(path: Path) -> str:
     return hashlib.sha256(path.read_bytes()).hexdigest()
 
 
+def reference_present() -> bool:
+    """Whether the reference checkout can be read by this user (a stat() of a path it cannot traverse would raise)."""
+    return os.access(REFERENCE / "aurora", os.R_OK | os.X_OK)
+
+
 def build(force: bool = False) -> Path:
     src = REFERENCE / "aurora"
-    if not src.is_dir():
+    if not reference_present():
         if (OUT / "aurora" / "__init__.py").exists():
             return OUT  # GPU box: use what travelled with the snapshot
         raise FileNotFoundError(f"{src} not found and {OUT} was not built; run oracle/build_ref.py in the build container")

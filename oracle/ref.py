@@ -18,7 +18,9 @@ REF_DIR = HERE / "_ref"
 
 
 def available() -> bool:
-    return (REF_DIR / "aurora" / "__init__.py").exists() or Path("/root/reference/aurora").is_dir()
+    from oracle import build_ref
+
+    return (REF_DIR / "aurora" / "__init__.py").exists() or build_ref.reference_present()
 
 
 def load():

@@ -9,6 +9,7 @@ and by the tests themselves (here and on the GPU box), so both sides see identic
 from __future__ import annotations
 
 import dataclasses
+import hashlib
 import math
 from datetime import datetime, timedelta
 
@@ -227,6 +228,13 @@ def tol_for(name: str) -> float:
 def rel_mean_abs(out: torch.Tensor, ref: torch.Tensor) -> float:
     """The reference's own acceptance metric: mean|out - ref| / mean|ref| (tests/test_model.py:45-61)."""
     return float((out.double() - ref.double()).abs().mean() / ref.double().abs().mean().clamp_min(1e-30))
+
+
+def array_digest(a) -> list:
+    """[shape, dtype, SHA-256 of the bytes] of a tensor or array: stored in place of a reference output, it still
+    compares bit for bit."""
+    a = np.ascontiguousarray(a.detach().cpu().numpy() if torch.is_tensor(a) else a)
+    return [list(a.shape), str(a.dtype), hashlib.sha256(a.tobytes()).hexdigest()]
 
 
 def field_error(out: torch.Tensor, ref: torch.Tensor, angle: bool = False) -> tuple[float, float]:

@@ -1,19 +1,28 @@
 """Generate the golden fixtures in this directory by running the UNMODIFIED reference
-(/root/reference, imported through the 4-symbol timm stand-in in tests/_shims) on the deterministic
-inputs of tests/fixtures.py.  Run in the build container only (the GPU box has no /root/reference):
+(a checkout of microsoft/aurora, imported through the 4-symbol timm stand-in in tests/_shims) on the
+deterministic inputs of tests/fixtures.py:
 
-    PYTHONPATH=/root/reference:tests/_shims:. python tests/golden/make_golden.py
+    PYTHONPATH=<reference checkout>:tests/_shims:. python tests/golden/make_golden.py [what ...]
+
+`fullsize` needs a B200; `oracle/_ref` (made by oracle/build_ref.py) holds the reference and the stand-in:
+
+    PYTHONPATH=oracle/_ref:. python tests/golden/make_golden.py fullsize
 
 Outputs
     windows.npz        gather indices and mask group ids of roll->pad->window_partition_3d and
                        compute_3d_shifted_window_mask for the shape cases of SURVEY.md App. A.5
+    windows_random.json  SHA-256 digests of the same maps on the random geometries of test_windows_random_cpu.py
     model_<case>.npz   float32 copies of the reference's float64 forward outputs (+ encoder / backbone taps)
     keys.json          state_dict key -> shape for the reference presets (parameter-layout parity)
+    batch_reference.json, regrid_reference.npz   the reference's `Batch` transforms (test_batch_host.py)
+    fullsize_<case>.npz  the reference's full-size forwards on a B200, sampled (test_fullsize_e2e_gpu.py)
 """
 
 import dataclasses
+import gc
 import hashlib
 import json
+import math
 import sys
 import types
 from pathlib import Path
@@ -169,12 +178,169 @@ def gen_compat():
     print("compat.json", {k: len(v) for k, v in out.items()})
 
 
+def gen_windows_random():
+    """roll -> pad -> window_partition_3d and compute_3d_shifted_window_mask of the reference on the random geometries
+    of test_windows_random_cpu.py, as digests of the arrays that test compares."""
+    from tests import test_windows_random_cpu as T
+
+    out = {}
+    for chunk in range(T.REFERENCE_CHUNKS):
+        recs = []
+        for res, shifted, warped in T._geometries(30, 200 + chunk):
+            c, h, w = res
+            ss0 = tuple(s // 2 for s in WS0) if shifted else (0, 0, 0)
+            ws, ss = maybe_adjust_windows(WS0, ss0, res)
+            x = (torch.arange(c * h * w, dtype=torch.float64) + 1).view(1, c, h, w, 1)
+            if any(ss):
+                x = torch.roll(x, shifts=(-ss[0], -ss[1], -ss[2]), dims=(1, 2, 3))
+            x = ref_swin.pad_3d(x, ((-c) % ws[0], (-h) % ws[1], (-w) % ws[2]))
+            idx = ref_swin.window_partition_3d(x, ws).reshape(-1, ws[0] * ws[1] * ws[2]).long().numpy() - 1
+            rec = {"res": list(res), "shifted": shifted, "warped": warped, "shift_after_adjust": any(ss),
+                   "idx": fx.array_digest(idx.astype(np.int32))}
+            if any(ss):
+                ref_swin.compute_3d_shifted_window_mask.cache_clear()
+                try:
+                    mask, img = ref_swin.compute_3d_shifted_window_mask(c, h, w, ws, ss, torch.device("cpu"),
+                                                                        torch.float32, warped)
+                except RuntimeError:  # the reference's own `.view` fails on some degenerate grids (swin3d.py:355)
+                    rec["mask"] = None
+                else:
+                    grp = ref_swin.window_partition_3d(img, ws).reshape(-1, ws[0] * ws[1] * ws[2]).to(torch.uint8)
+                    same = grp[:, :, None] == grp[:, None, :]
+                    assert fx.array_digest(mask) == fx.array_digest(torch.where(same, 0.0, -100.0)), res
+                    rec["grp"], rec["mask"] = fx.array_digest(grp), fx.array_digest(mask)
+            recs.append(rec)
+        out[str(chunk)] = recs
+    (HERE / "windows_random.json").write_text(json.dumps(out, indent=0))
+    print("windows_random.json", sum(len(v) for v in out.values()), "geometries")
+
+
+REGRID_SAMPLES = 256  # points per regridded field; the whole field enters through its sum
+
+
+def gen_batch():
+    """The reference's normalisation constants and `Batch` normalise / unnormalise / crop / regrid on the inputs of
+    test_batch_host.py."""
+    from aurora import normalisation as rn
+
+    from tests import test_batch_host as T
+
+    rb = to_ref_batch(T.transforms_batch())
+    transforms = {"normalise": rb.normalise(surf_stats={}), "unnormalise": rb.normalise(surf_stats={}).unnormalise(surf_stats={}),
+                  "crop3": rb.crop(3)}
+    assert sorted(transforms) == sorted(T.batch_transforms(T.transforms_batch()))
+    out = {"locations": {k: float(v) for k, v in rn.locations.items()},
+           "scales": {k: float(v) for k, v in rn.scales.items()}, "transforms": {}}
+    for name, b in transforms.items():
+        rec = {"spatial_shape": list(b.spatial_shape), "lat": fx.array_digest(b.metadata.lat)}
+        for grp in T.GROUPS:
+            rec[grp] = {k: fx.array_digest(v) for k, v in getattr(b, grp).items()}
+        out["transforms"][name] = rec
+    (HERE / "batch_reference.json").write_text(json.dumps(out, indent=0))
+
+    rng = np.random.Generator(np.random.PCG64(0))
+    rb = to_ref_batch(T.regrid_batch())
+    arrays = {}
+    for res in T.REGRID_RES:
+        b, tag = rb.regrid(res), T.regrid_tag(res)
+        arrays[f"{tag}.spatial_shape"] = np.array(b.spatial_shape)
+        arrays[f"{tag}.lat"], arrays[f"{tag}.lon"] = b.metadata.lat.numpy(), b.metadata.lon.numpy()
+        for grp in T.GROUPS:
+            g, fields = grp.split("_")[0], getattr(b, grp)
+            arrays.update(sampled_fields(f"{tag}.{g}", fields, REGRID_SAMPLES, rng))
+            arrays[f"{tag}.{g}.vmax"] = np.array([float(v.abs().max()) for v in fields.values()])
+            arrays[f"{tag}.{g}.sum"] = np.array([float(v.double().sum()) for v in fields.values()])
+    np.savez_compressed(HERE / "regrid_reference.npz", **arrays)
+    print("batch_reference.json, regrid_reference.npz", len(arrays), "arrays")
+
+
+def sampled_fields(prefix: str, fields: dict, n: int, rng) -> dict:
+    """Fields of one shape at up to `n` fixed random points: `<prefix>.names`, `.shape`, `.idx` (sorted flat indices),
+    `.val` (one row per field, float32)."""
+    (shape,) = {tuple(v.shape) for v in fields.values()}
+    assert math.prod(shape) < 2**31, shape
+    idx = np.unique(rng.integers(0, math.prod(shape), n)).astype(np.int32)
+    rows = [v.reshape(-1)[torch.from_numpy(idx).long().to(v.device)].float().cpu().numpy() for v in fields.values()]
+    return {f"{prefix}.names": np.array(list(fields)), f"{prefix}.shape": np.array(shape), f"{prefix}.idx": idx,
+            f"{prefix}.val": np.stack(rows)}
+
+
+# points per field (2 KiB each): on a B200 the rel-mean-abs error at these points came within 20 % of the whole-field
+# value for every field of the four cases, each at least a third inside its bound
+FULLSIZE_SAMPLES = 512
+
+
+def gen_fullsize(only=None):
+    """The reference's full-size forwards for test_fullsize_e2e_gpu.py, on a B200: fp32 with TF32 off and its own
+    autocast recipe, on that test's inputs.  Stores the fp32 outputs and backbone output at a fixed sample of points,
+    mean |fp32| of every whole field and the spread autocast vs fp32 over every whole field; prints our error over the
+    whole field next to the one at the stored points."""
+    import bench
+    from tests import test_fullsize_e2e_gpu as T
+
+    torch.backends.cuda.matmul.allow_tf32 = False
+    torch.backends.cudnn.allow_tf32 = False  # conv3d patch embedding of the reference in true fp32
+    rng = np.random.Generator(np.random.PCG64(0))
+    for case in sorted(T.CASES):
+        if only and not any(case.startswith(o) for o in only):
+            continue
+        ours, tap_ours = T.run_ours(case)[:2]
+        ours[("tap", "backbone")] = tap_ours
+        model, dev_batch = T.make_inputs(case)
+        sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
+        del model
+        rb = to_ref_batch(dev_batch)
+        runs = {}
+        for tag, autocast in (("fp32", False), ("autocast", True)):
+            with torch.device("cuda"):
+                rmodel = getattr(aurora, bench.WORKLOADS[T.CASES[case]][0])(autocast=autocast)
+            rmodel.load_state_dict(sd, strict=True)
+            rmodel = rmodel.eval()
+            taps = {}
+            hook = rmodel.backbone.register_forward_hook(lambda m, i, o: taps.__setitem__("tap", o.detach().float()[0]))
+            with torch.inference_mode():
+                rp = rmodel.forward(rb)
+            hook.remove()
+            torch.cuda.synchronize()
+            fields = {("surf", k): v for k, v in rp.surf_vars.items()}
+            fields.update({("atmos", k): v for k, v in rp.atmos_vars.items()})
+            fields[("tap", "backbone")] = taps["tap"]
+            runs[tag] = fields, rp.metadata
+            del rp, rmodel
+            gc.collect()
+            torch.cuda.empty_cache()
+        ref, meta = runs["fp32"]
+        out = {"meta.time0": np.array(meta.time[0].timestamp()), "meta.rollout_step": np.array(meta.rollout_step),
+               "meta.atmos_levels": np.array(meta.atmos_levels)}
+        print(f"[fullsize golden] {case}")
+        for group in ("surf", "atmos", "tap"):
+            fields = {k: v for (g, k), v in ref.items() if g == group}
+            out.update(sampled_fields(group, fields, FULLSIZE_SAMPLES, rng))
+            out[f"{group}.absmean"] = np.array([v.double().abs().mean().item() for v in fields.values()])
+            out[f"{group}.spread"] = np.array([fx.rel_mean_abs(runs["autocast"][0][(group, k)], v) for k, v in fields.items()])
+            for row, (k, v) in enumerate(fields.items()):
+                whole = fx.rel_mean_abs(ours[(group, k)], v)
+                print(f"  {group:5s} {k:8s} ours: whole field {whole:.3e}, at the stored points "
+                      f"{T.sampled_rel(ours[(group, k)], out, group, row):.3e}   reference autocast {out[f'{group}.spread'][row]:.3e}")
+        del runs, ref, ours
+        gc.collect()
+        torch.cuda.empty_cache()
+        np.savez_compressed(HERE / f"fullsize_{case}.npz", **out)
+
+
 if __name__ == "__main__":
-    only = [a.split("=", 1)[1] for a in sys.argv[1:] if a.startswith("--only=")]  # model case name prefixes
-    what = [a for a in sys.argv[1:] if not a.startswith("--only=")] or ["windows", "models", "rollout", "keys", "compat"]
+    only = [a.split("=", 1)[1] for a in sys.argv[1:] if a.startswith("--only=")]  # model / full-size case name prefixes
+    what = [a for a in sys.argv[1:] if not a.startswith("--only=")] or ["windows", "windows_random", "models", "rollout",
+                                                                         "keys", "compat", "batch"]
     torch.manual_seed(0)
     if "windows" in what:
         gen_windows()
+    if "windows_random" in what:
+        gen_windows_random()
+    if "batch" in what:
+        gen_batch()
+    if "fullsize" in what:
+        gen_fullsize(only)
     if "models" in what:
         gen_models(only)
     if "rollout" in what:

@@ -1,11 +1,13 @@
 """`Batch` / `Metadata` host logic (no GPU): validation and error behaviour of `aurora/batch.py:24-190`, the
-normalisation constants of `aurora/normalisation.py`, and — when the reference checkout is present (build
-container only) — a live cross-check of normalise / unnormalise / crop against the reference classes."""
+normalisation constants of `aurora/normalisation.py`, and normalise / unnormalise / crop / regrid against what the
+reference classes computed on the same inputs (tests/golden/batch_reference.json and regrid_reference.npz, written by
+make_golden.py)."""
 
-import sys
+import json
 from datetime import datetime
 from pathlib import Path
 
+import numpy as np
 import pytest
 import torch
 
@@ -13,7 +15,8 @@ from aurora_b200 import Batch, Metadata
 from aurora_b200 import stats
 from tests import fixtures as fx
 
-REF = Path("/root/reference")
+GOLD = Path(__file__).parent / "golden"
+GROUPS = ("surf_vars", "static_vars", "atmos_vars")
 
 
 def _meta(h=17, w=32, **kw):
@@ -69,31 +72,28 @@ def test_normalise_roundtrip_and_overrides():
     assert stats.level_to_str(850) == "850" and stats.level_to_str(12.5) == "12_5"
 
 
-@pytest.mark.skipif(not REF.exists(), reason="reference checkout not present (GPU box)")
+def batch_transforms(b):
+    """The transforms of `test_against_reference_classes_live`, by the name they are stored under."""
+    return {"normalise": b.normalise(), "unnormalise": b.normalise().unnormalise(), "crop3": b.crop(3)}
+
+
+def transforms_batch():
+    return fx.make_batch(fx.CONFIGS["tiny_air"], 46, 90, levels=fx.LEVELS13, b=2)
+
+
 def test_against_reference_classes_live():
-    sys.path[:0] = [str(REF), str(Path(__file__).parent / "_shims")]
-    try:
-        import aurora
-        from aurora import normalisation as rn
-    finally:
-        del sys.path[:2]
+    gold = json.loads((GOLD / "batch_reference.json").read_text())
     # every normalisation constant of the reference is in our table, bit for bit as float64
-    assert stats.locations == {k: float(v) for k, v in rn.locations.items()}
-    assert stats.scales == {k: float(v) for k, v in rn.scales.items()}
-    cfg = fx.CONFIGS["tiny_air"]
-    b = fx.make_batch(cfg, 46, 90, levels=fx.LEVELS13, b=2)
-    rb = aurora.Batch(dict(b.surf_vars), dict(b.static_vars), dict(b.atmos_vars),
-                      aurora.Metadata(lat=b.metadata.lat, lon=b.metadata.lon, time=b.metadata.time,
-                                      atmos_levels=b.metadata.atmos_levels))
-    for ours, ref in ((b.normalise(), rb.normalise(surf_stats={})),
-                      (b.normalise().unnormalise(), rb.normalise(surf_stats={}).unnormalise(surf_stats={})),
-                      (b.crop(3), rb.crop(3))):
-        assert ours.spatial_shape == tuple(ref.spatial_shape)
-        for grp in ("surf_vars", "static_vars", "atmos_vars"):
-            assert list(getattr(ours, grp)) == list(getattr(ref, grp))
-            for k, v in getattr(ref, grp).items():
-                assert torch.equal(getattr(ours, grp)[k], v), (grp, k)
-        assert torch.equal(ours.metadata.lat, ref.metadata.lat)
+    assert stats.locations == gold["locations"]
+    assert stats.scales == gold["scales"]
+    for name, ours in batch_transforms(transforms_batch()).items():
+        ref = gold["transforms"][name]
+        assert list(ours.spatial_shape) == ref["spatial_shape"], name
+        for grp in GROUPS:
+            assert list(getattr(ours, grp)) == list(ref[grp]), (name, grp)
+            for k, digest in ref[grp].items():
+                assert fx.array_digest(getattr(ours, grp)[k]) == digest, (name, grp, k)
+        assert fx.array_digest(ours.metadata.lat) == ref["lat"], name
 
 
 def test_regrid_properties():
@@ -118,27 +118,42 @@ def test_regrid_properties():
     assert torch.allclose(fine.surf_vars["2t"][..., ::2, ::2], b.surf_vars["2t"], rtol=5e-6, atol=1e-4)
 
 
-@pytest.mark.skipif(not REF.exists(), reason="reference checkout not present (GPU box)")
-@pytest.mark.parametrize("res", [5.0, 11.25, 7.3])
+REGRID_RES = (5.0, 11.25, 7.3)
+
+
+def regrid_tag(res: float) -> str:
+    return str(res).replace(".", "p")
+
+
+def regrid_batch():
+    return fx.make_batch(fx.CONFIGS["tiny"], 17, 32, levels=fx.LEVELS4, b=2)
+
+
+@pytest.mark.parametrize("res", REGRID_RES)
 def test_regrid_against_reference_live(res):
-    sys.path[:0] = [str(REF), str(Path(__file__).parent / "_shims")]
-    try:
-        import aurora
-    finally:
-        del sys.path[:2]
-    cfg = fx.CONFIGS["tiny"]
-    b = fx.make_batch(cfg, 17, 32, levels=fx.LEVELS4, b=2)
-    rb = aurora.Batch(dict(b.surf_vars), dict(b.static_vars), dict(b.atmos_vars),
-                      aurora.Metadata(lat=b.metadata.lat, lon=b.metadata.lon, time=b.metadata.time,
-                                      atmos_levels=b.metadata.atmos_levels))
-    ours, ref = b.regrid(res), rb.regrid(res)
-    assert ours.spatial_shape == tuple(ref.spatial_shape)
-    assert torch.allclose(ours.metadata.lat, ref.metadata.lat, atol=1e-12) and torch.allclose(ours.metadata.lon, ref.metadata.lon, atol=1e-12)
-    for grp in ("surf_vars", "static_vars", "atmos_vars"):
-        for k, v in getattr(ref, grp).items():
-            got = getattr(ours, grp)[k]
-            assert got.dtype == torch.float32 and got.shape == v.shape
-            assert torch.allclose(got, v, rtol=2e-6, atol=1e-6 * float(v.abs().max())), (grp, k, float((got - v).abs().max()))
+    """The reference's regridded fields are stored at a fixed sample of points, with their max |value| and their sum:
+    every stored point within the tolerance below, and the sum over the whole field within the sum of those bounds."""
+    gold = np.load(GOLD / "regrid_reference.npz")
+    tag = regrid_tag(res)
+    ours = regrid_batch().regrid(res)
+    assert list(ours.spatial_shape) == gold[f"{tag}.spatial_shape"].tolist()
+    assert torch.allclose(ours.metadata.lat, torch.from_numpy(gold[f"{tag}.lat"]), atol=1e-12)
+    assert torch.allclose(ours.metadata.lon, torch.from_numpy(gold[f"{tag}.lon"]), atol=1e-12)
+    for grp in GROUPS:
+        g, fields = grp.split("_")[0], getattr(ours, grp)
+        names = gold[f"{tag}.{g}.names"].tolist()
+        assert sorted(names) == sorted(fields), grp
+        idx = torch.from_numpy(gold[f"{tag}.{g}.idx"].astype(np.int64))
+        for row, k in enumerate(names):
+            got = fields[k]
+            assert got.dtype == torch.float32 and list(got.shape) == gold[f"{tag}.{g}.shape"].tolist(), (grp, k)
+            v = torch.from_numpy(gold[f"{tag}.{g}.val"][row])
+            vmax = float(gold[f"{tag}.{g}.vmax"][row])
+            atol, rtol = 1e-6 * vmax, 2e-6
+            sample = got.reshape(-1)[idx]
+            assert torch.allclose(sample, v, rtol=rtol, atol=atol), (grp, k, float((sample - v).abs().max()))
+            total = float(got.double().sum()) - float(gold[f"{tag}.{g}.sum"][row])
+            assert abs(total) <= got.numel() * (atol + rtol * vmax), (grp, k, total)
 
 
 def test_netcdf_io_needs_xarray_like_the_reference(tmp_path):
